@@ -2,7 +2,7 @@
 """
 bench.py -- headline benchmark of the compress/decompress hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--layers L]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--layers L] [--dump-outputs DIR]
 
 Workload (configs[1] of BASELINE.json): W4A16 group_size=128 quantize + pack_to_int32 over every
 Linear weight of a Llama-3-8B-shaped model (32 layers x {q,k,v,o,gate,up,down} = 224 bf16 tensors,
@@ -243,6 +243,8 @@ def run_b200(a):
     ms = time_steps(step, a.steps, a.warmup, dist_on, sampler=cs)
     launches = (N.launch_count() - l0) - a.warmup  # one launch per step
     verified, verified_idx = (verify_timed_outputs(ws, scs, outs) if rank == 0 else (None, None))
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, outs)
     clocks = cs.summary()
     ms_per_step = ms / a.steps
     value = world * weight_bytes / (ms_per_step * 1e-3) / 1e9
@@ -647,6 +649,29 @@ def verify_timed_outputs(ws, scs, outs):
     return ok, picks
 
 
+DUMP_WORDS_PER_TENSOR = 8192
+DUMP_SEED = 0
+
+
+def dump_outputs(directory: str, outs):
+    """What the last timed step wrote, for comparing two builds output for output: the packed int32 words at the same seeded
+    positions of every tensor (all 3.5 GB would not fit a 64 MB dump).  Written as float64, which holds every int32 exactly:
+      weight_packed_sample.npy        [tensors, DUMP_WORDS_PER_TENSOR]  the sampled words
+      weight_packed_sample_index.npy  [tensors, DUMP_WORDS_PER_TENSOR]  their flat positions in each [rows, cols / 8] output"""
+    import numpy as np
+
+    g = torch.Generator().manual_seed(DUMP_SEED)
+    words, index = [], []
+    for o in outs:
+        n = min(DUMP_WORDS_PER_TENSOR, o.numel())
+        idx = torch.randint(0, o.numel(), (n,), generator=g).sort().values
+        words.append(o.reshape(-1)[idx.to(o.device)].cpu().double())
+        index.append(idx.double())
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "weight_packed_sample.npy"), torch.stack(words).numpy())
+    np.save(os.path.join(directory, "weight_packed_sample_index.npy"), torch.stack(index).numpy())
+
+
 def run_e2e(ws, scs, a, dist_on, world, outs=None):
     """The same pass end to end through the public API: ModelCompressor.compress_model() on a HOST-resident
     model (pinned weights and scales), i.e. the call llm-compressor makes before save_pretrained.  Every step
@@ -936,7 +961,11 @@ def main():
     ap.add_argument("--cfg5", action="store_true", help="run the sharded leg even with one rank (under a 1-rank torchrun; pick --cfg5-layers <= 40)")
     ap.add_argument("--cfg5-layers", type=int, default=80, help="Llama-3-70B layers of the sharded leg (80 = the full model, 560 tensors)")
     ap.add_argument("--cfg5-reps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write a seeded sample of the last step's packed words to DIR/*.npy (float64)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.warmup < 3:
         a.warmup = 3
     if a.impl == "cpu-worker":

@@ -16,6 +16,7 @@ copied into this repository; only tensors produced by running it are stored.
 Everything stored is a plain dict of tensors / python scalars, loadable with
 torch.load(weights_only=True).
 """
+import glob
 import os
 import shutil
 import sys
@@ -62,17 +63,37 @@ from compressed_tensors.utils import semi_structured_conversions as ssc  # noqa:
 from compressed_tensors.utils.permutations_24 import get_permutations_24  # noqa: E402
 
 
-def save(name, obj):
-    """gzip-compressed torch.save (load with tests/golden/__init__.py:load)"""
-    import gzip
-    import io
+MAX_FILE_BYTES = 1 << 20
 
-    path = os.path.join(HERE, name + ".gz")
-    buf = io.BytesIO()
-    torch.save(obj, buf)
-    with gzip.GzipFile(path, "wb", compresslevel=9, mtime=0) as f:
-        f.write(buf.getvalue())
-    print(f"{name}: {os.path.getsize(path) / 1024:.0f} KiB, {len(obj) if hasattr(obj, '__len__') else ''} entries")
+
+def save(name, obj):
+    """xz-compressed torch.save (load with tests/golden/__init__.py:load); a list of cases that would pass MAX_FILE_BYTES is written in
+    parts <stem>.<i>.pt.xz of consecutive cases"""
+    import io
+    import lzma
+
+    def encode(o):
+        buf = io.BytesIO()
+        torch.save(o, buf)
+        return lzma.compress(buf.getvalue(), preset=9 | lzma.PRESET_EXTREME)
+
+    stem = name[: -len(".pt")]
+    data = encode(obj)
+    chunks = [(stem + ".pt.xz", data)]
+    k = 1
+    while max(len(d) for _, d in chunks) > MAX_FILE_BYTES:
+        if not isinstance(obj, list) or k >= len(obj):
+            raise ValueError(f"{name}: {len(data)} bytes compressed, more than {MAX_FILE_BYTES}")
+        k += 1
+        step = -(-len(obj) // k)
+        chunks = [(f"{stem}.{i}.pt.xz", encode(obj[j:j + step])) for i, j in enumerate(range(0, len(obj), step))]
+    for old in [stem + ".pt.gz", stem + ".pt.xz"] + [os.path.basename(p) for p in glob.glob(os.path.join(HERE, stem + ".*.pt.xz"))]:
+        if os.path.exists(os.path.join(HERE, old)):
+            os.remove(os.path.join(HERE, old))
+    for fname, d in chunks:
+        with open(os.path.join(HERE, fname), "wb") as f:
+            f.write(d)
+        print(f"{fname}: {len(d) / 1024:.0f} KiB")
 
 
 # --------------------------------------------------------------------------- #

@@ -1,8 +1,9 @@
 """
-Differential fuzz of the host mirror against the reference itself (TEST INFRASTRUCTURE; build container only: it imports the
-reference from /root/reference through tests/golden/make_golden.py's temporary copy, next to compressed_tensors_b200 in one process).
+Differential fuzz of the host mirror against the reference itself (TEST INFRASTRUCTURE), on seeded cases, against the reference's
+outcomes recorded in tests/golden/reference_fuzz/fuzz_host_mirror.json (recorded.py; `--record` re-records them, importing the
+reference through tests/golden/make_golden.py).
 
-    python tests/reference_compat/fuzz_host_mirror.py [iterations]
+    python tests/reference_compat/fuzz_host_mirror.py [iterations] [--record]
 
 Three parts, each compares outcome AND exception type:
   args     random QuantizationArgs keyword sets (valid and invalid)            -> model_dump()
@@ -18,16 +19,20 @@ import warnings
 warnings.filterwarnings("ignore")
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-sys.path[:0] = [os.path.join(ROOT, "tests", "golden"), ROOT]
+sys.path[:0] = [HERE, os.path.join(ROOT, "tests", "golden"), ROOT]
 from loguru import logger  # noqa: E402
 
 logger.remove()
-import make_golden as mg  # noqa: E402,F401  (imports the reference as `compressed_tensors` from a temp copy)
 import torch  # noqa: E402
 
-import compressed_tensors.quantization as R  # noqa: E402
-import compressed_tensors.quantization.quant_scheme as RS  # noqa: E402
-from compressed_tensors.quantization.utils import calculate_qparams as rq, compute_dynamic_scales_and_zp as rd, generate_gparam as rg  # noqa: E402
+from recorded import Reference, evaluate, values_of  # noqa: E402
+
+REF = Reference("fuzz_host_mirror")
+if REF.recording:
+    import make_golden as mg  # noqa: E402,F401  (imports the reference as `compressed_tensors` from a temp copy)
+    import compressed_tensors.quantization as R  # noqa: E402
+    import compressed_tensors.quantization.quant_scheme as RS  # noqa: E402
+    from compressed_tensors.quantization.utils import calculate_qparams as rq, compute_dynamic_scales_and_zp as rd, generate_gparam as rg  # noqa: E402
 
 import compressed_tensors_b200.quantization as M  # noqa: E402
 import compressed_tensors_b200.quantization.quant_scheme as MS  # noqa: E402
@@ -45,13 +50,6 @@ def norm(v):
     return str(v) if isinstance(v, torch.dtype) else v
 
 
-def outcome(fn):
-    try:
-        return ("ok", fn())
-    except Exception as e:  # noqa: BLE001
-        return ("err", type(e).__name__)
-
-
 def fuzz_args(n):
     rnd = random.Random(0)
     space = dict(
@@ -63,8 +61,8 @@ def fuzz_args(n):
     bad = 0
     for _ in range(n):
         kw = {k: rnd.choice(v) for k, v in space.items() if rnd.random() < 0.6}
-        r = outcome(lambda: (lambda a: (norm(a.model_dump()), str(a.pytorch_dtype())))(R.QuantizationArgs(**kw)))
-        m = outcome(lambda: (lambda a: (norm(a.model_dump()), str(a.pytorch_dtype())))(M.QuantizationArgs(**kw)))
+        r = REF("args", lambda: (lambda a: (norm(a.model_dump()), str(a.pytorch_dtype())))(R.QuantizationArgs(**kw)))
+        m = evaluate(lambda: (lambda a: (norm(a.model_dump()), str(a.pytorch_dtype())))(M.QuantizationArgs(**kw)))
         if r != m:
             bad += 1
             if bad <= 5:
@@ -75,12 +73,12 @@ def fuzz_args(n):
 def fuzz_schemes(n):
     bad = 0
     checked = 0
-    if set(RS.PRESET_SCHEMES) != set(MS.PRESET_SCHEMES):
+    if REF("presets", lambda: sorted(RS.PRESET_SCHEMES)) != evaluate(lambda: sorted(MS.PRESET_SCHEMES)):
         bad += 1
-        print("PRESET NAMES", sorted(set(RS.PRESET_SCHEMES) ^ set(MS.PRESET_SCHEMES)))
-    for name in sorted(set(RS.PRESET_SCHEMES) & set(MS.PRESET_SCHEMES)):
+        print("PRESET NAMES differ")
+    for name in sorted(MS.PRESET_SCHEMES):
         checked += 1
-        if norm(R.preset_name_to_scheme(name, ["Linear"]).model_dump()) != norm(M.preset_name_to_scheme(name, ["Linear"]).model_dump()):
+        if REF("presets", lambda: norm(R.preset_name_to_scheme(name, ["Linear"]).model_dump())) != evaluate(lambda: norm(M.preset_name_to_scheme(name, ["Linear"]).model_dump())):
             bad += 1
             print("PRESET", name)
     rnd = random.Random(1)
@@ -100,22 +98,20 @@ def fuzz_schemes(n):
         fmt = rnd.choice([None, "pack-quantized", "int-quantized", "float-quantized", "nvfp4-pack-quantized", "dense", "bogus"])
 
         def run(Q):
-            return outcome(lambda: norm(Q.QuantizationScheme(targets=["Linear"], format=fmt, **{k: (Q.QuantizationArgs(**v) if v else None) for k, v in parts.items()}).model_dump()))
+            return norm(Q.QuantizationScheme(targets=["Linear"], format=fmt, **{k: (Q.QuantizationArgs(**v) if v else None) for k, v in parts.items()}).model_dump())
 
         checked += 1
-        r, m = run(R), run(M)
+        r, m = REF("schemes", lambda: run(R)), evaluate(lambda: run(M))
         if r != m:
             bad += 1
             if bad <= 5:
-                print("SCHEME", parts, fmt, "\n  reference", r[0], r[1] if r[0] == "err" else "", "\n  mirror   ", m[0], m[1] if m[0] == "err" else "")
+                print("SCHEME", parts, fmt, "\n  reference", r, "\n  mirror   ", m)
     return checked, bad
 
 
-def same(a, b):
-    if a.dtype != b.dtype or a.shape != b.shape:
-        return False
-    a, b = (a.view(torch.uint8), b.view(torch.uint8)) if a.dtype == FP8 else (a, b)
-    return torch.equal(a, b) or (a.is_floating_point() and torch.equal(torch.nan_to_num(a.float(), nan=7.0), torch.nan_to_num(b.float(), nan=7.0)))
+def same_values(pair):
+    """qparams compare like torch.equal, NaN standing for itself (fp8 by bits)"""
+    return [values_of(t.view(torch.uint8)) if t.dtype == FP8 else values_of(t) for t in pair]
 
 
 def fuzz_qparams(n):
@@ -127,9 +123,6 @@ def fuzz_qparams(n):
             dict(num_bits=4, type="float", symmetric=True, strategy="group", group_size=32, scale_dtype=torch.uint8, zp_dtype=torch.uint8),
             dict(num_bits=8, type="float", symmetric=True, strategy="group", group_size=32, scale_dtype=torch.uint8, zp_dtype=torch.uint8)]
     bad = checked = 0
-
-    def differs(r, m):
-        return r[0] != m[0] or (r[0] == "err" and r[1] != m[1]) or (r[0] == "ok" and not (same(r[1][0], m[1][0]) and same(r[1][1], m[1][1])))
 
     for _ in range(n):
         kw = dict(rnd.choice(cfgs))
@@ -146,28 +139,28 @@ def fuzz_qparams(n):
             hi = torch.zeros_like(hi)
         gs = None
         if kw["strategy"] == "tensor_group":
-            a, b = rg(lo.min(), hi.max()), mgp(lo.min(), hi.max())
+            gs = mgp(lo.min(), hi.max())       # once it matches, bit-identical to the reference's
             checked += 1
-            if not same(a, b):
+            if REF("qparams", lambda: same_values([rg(lo.min(), hi.max())])) != evaluate(lambda: same_values([gs])):
                 bad += 1
-                print("GPARAM", lo.min(), hi.max(), a, b)
-            gs = a
+                print("GPARAM", lo.min(), hi.max(), gs)
         extra = dict(global_scale=gs) if gs is not None else {}
-        r, m = outcome(lambda: rq(lo, hi, R.QuantizationArgs(**kw), **extra)), outcome(lambda: mq(lo, hi, M.QuantizationArgs(**kw), **extra))
+        r = REF("qparams", lambda: same_values(rq(lo, hi, R.QuantizationArgs(**kw), **extra)))
+        m = evaluate(lambda: same_values(mq(lo, hi, M.QuantizationArgs(**kw), **extra)))
         checked += 1
-        if differs(r, m):
+        if r != m:
             bad += 1
             if bad <= 5:
-                print("QPARAMS", kw, dt, shape, r[0], m[0])
+                print("QPARAMS", kw, dt, shape, r, m)
         x = (torch.randn(rnd.choice([(2, 3, 64), (4, 64), (64,)]), generator=g) * mag).to(dt)
         kd = dict(kw, dynamic=True)
-        r = outcome(lambda: rd(value=x, args=R.QuantizationArgs(**kd), module=torch.nn.Identity(), **extra))
-        m = outcome(lambda: md(value=x, args=M.QuantizationArgs(**kd), module=torch.nn.Identity(), **extra))
+        r = REF("qparams", lambda: same_values(rd(value=x, args=R.QuantizationArgs(**kd), module=torch.nn.Identity(), **extra)))
+        m = evaluate(lambda: same_values(md(value=x, args=M.QuantizationArgs(**kd), module=torch.nn.Identity(), **extra)))
         checked += 1
-        if differs(r, m):
+        if r != m:
             bad += 1
             if bad <= 5:
-                print("DYNAMIC", kd, dt, tuple(x.shape), r[0], m[0])
+                print("DYNAMIC", kd, dt, tuple(x.shape), r, m)
     return checked, bad
 
 
@@ -178,6 +171,7 @@ def main():
         checked, bad = fn(k)
         total_bad += bad
         print(f"{name}: {checked} checked, {bad} mismatches", flush=True)
+    total_bad += REF.finish()
     sys.exit(1 if total_bad else 0)
 
 

@@ -1,11 +1,13 @@
 """
-Differential fuzz of `ModelCompressor` against the reference's (TEST INFRASTRUCTURE; build container only): the same random small model and
+Differential fuzz of `ModelCompressor` against the reference's (TEST INFRASTRUCTURE): the same seeded random small model and
 quantization config go through apply_quantization_config -> (identical qparams) -> ModelCompressor.from_pretrained_model ->
-compress_model -> update_config -> decompress_model in the reference (imported as `compressed_tensors` from a temporary copy) and in
-this package (its tensor-level front end rebound to the CPU oracle).  Compared: every module's state dict after compress (keys, dtypes,
-shapes, bits), the `quantization_config` written to config.json, and every module's state dict after decompress.
+compress_model -> update_config -> decompress_model in this package (its tensor-level front end rebound to the CPU oracle), against
+the reference's outcomes recorded in tests/golden/reference_fuzz/fuzz_model_compressor.json (recorded.py; `--record` re-records them,
+importing the reference as `compressed_tensors` through tests/golden/make_golden.py).  Compared: every module's state dict after
+initialisation, after compress (keys, dtypes, shapes, bits), the `quantization_config` written to config.json, and every module's state
+dict after decompress.
 
-    python tests/reference_compat/fuzz_model_compressor.py [models]
+    python tests/reference_compat/fuzz_model_compressor.py [models] [--record]
 """
 import copy
 import json
@@ -22,22 +24,24 @@ sys.path[:0] = [HERE, os.path.join(ROOT, "tests", "golden"), ROOT]
 from loguru import logger  # noqa: E402
 
 logger.remove()
-import make_golden as mg  # noqa: E402,F401
 import torch  # noqa: E402
 
-import compressed_tensors as R  # noqa: E402
-import compressed_tensors.quantization as RQ  # noqa: E402
-from compressed_tensors.quantization.utils import calculate_qparams as r_qparams, generate_gparam as r_gparam  # noqa: E402
-from compressed_tensors.utils import get_direct_state_dict as r_state  # noqa: E402
+from recorded import Reference, evaluate  # noqa: E402
+
+REF = Reference("fuzz_model_compressor")
+if REF.recording:
+    import make_golden as mg  # noqa: E402,F401
+    import compressed_tensors as R  # noqa: E402
+    import compressed_tensors.quantization as RQ  # noqa: E402
+    from compressed_tensors.utils import get_direct_state_dict as r_state  # noqa: E402
 
 import oracle_patch  # noqa: E402
 
 oracle_patch.apply("compressed_tensors_b200")
 import compressed_tensors_b200 as M  # noqa: E402
 import compressed_tensors_b200.quantization as MQ  # noqa: E402
+from compressed_tensors_b200.quantization.utils import calculate_qparams as m_qparams, generate_gparam as m_gparam  # noqa: E402
 from compressed_tensors_b200.utils import get_direct_state_dict as m_state  # noqa: E402
-
-from fuzz_compressors import same_dict  # noqa: E402
 
 PRESETS = ["W4A16", "W4A16_ASYM", "W8A16", "W8A8", "W4A8", "FP8", "FP8_DYNAMIC", "FP8_BLOCK", "NVFP4A16", "NVFP4", "MXFP4A16", "MXFP4"]
 
@@ -54,7 +58,8 @@ def build(rnd, seed):
 
 
 def calibrate(model):
-    """memoryless min-max weights observer with the REFERENCE's rule; returns {module name: {param: tensor}} to load into both models"""
+    """memoryless min-max weights observer with the reference's rule (this package's calculate_qparams / generate_gparam, compared with
+    the reference's by fuzz_host_mirror.py); returns {module name: {param: tensor}} to load into both models"""
     out = {}
     for name, m in model.named_modules():
         scheme = getattr(m, "quantization_scheme", None)
@@ -76,9 +81,9 @@ def calibrate(model):
             lo, hi = blk.amin((1, 3)), blk.amax((1, 3))
         q = {}
         if s == "tensor_group":
-            gs = r_gparam(w.amin(), w.amax())
+            gs = m_gparam(w.amin(), w.amax())
             q["weight_global_scale"] = gs
-        sc, zp = r_qparams(lo, hi, a, global_scale=gs) if gs is not None else r_qparams(lo, hi, a)
+        sc, zp = m_qparams(lo, hi, a, global_scale=gs) if gs is not None else m_qparams(lo, hi, a)
         q["weight_scale"], q["weight_zero_point"] = sc, zp
         for base in ("input", "output"):        # static activation qparams are allocated uninitialised
             for suffix, val in (("scale", 0.5), ("zero_point", 0), ("global_scale", 2.0)):
@@ -99,13 +104,35 @@ def states(model, fn):
     return {n: {k: v for k, v in fn(m).items()} for n, m in model.named_modules()}
 
 
-def compare_models(a, b, what):
-    sa, sb = states(a, m_state), states(b, r_state)
-    for n in sb:
-        err = same_dict(sa.get(n, {}), sb[n], f"{what} {n or '<root>'}")
-        if err:
-            return err
-    return None
+def quantization_config(compressor):
+    with tempfile.TemporaryDirectory() as d:
+        compressor.update_config(d)
+        c = json.load(open(os.path.join(d, "config.json")))["quantization_config"]
+    c.pop("version", None)
+    return c
+
+
+def try_decompress(compressor, model, state):
+    try:
+        compressor.decompress_model(model)
+    except Exception:  # noqa: BLE001  (e.g. FP8_BLOCK with an [N, 1] scale grid: dequantize infers CHANNEL and the broadcast fails)
+        return "raised"       # both raising, whatever the exception, counts as agreement
+    return states(model, state)
+
+
+STAGES = ("initialized", "compressed", "config.json", "decompressed")
+
+
+def pipeline(pkg, model, q, state):
+    """the four stages of one case: module states after loading the qparams and after compress, the quantization_config, and the
+    outcome of decompress"""
+    load_qparams(model, q)
+    yield states(model, state)
+    compressor = pkg.ModelCompressor.from_pretrained_model(model)
+    compressor.compress_model(model)
+    yield states(model, state)
+    yield quantization_config(compressor)
+    yield try_decompress(compressor, model, state)
 
 
 def main():
@@ -116,50 +143,30 @@ def main():
         preset = rnd.choice(PRESETS)
         seed = rnd.randint(0, 10 ** 6)
         st = rnd.getstate()
-        ref_model = build(rnd, seed)
-        rnd.setstate(st)
         my_model = build(rnd, seed)
         cfg = dict(config_groups={preset: ["Linear"]}, ignore=["lm_head"])
-        RQ.apply_quantization_config(ref_model, RQ.QuantizationConfig(**cfg))
         MQ.apply_quantization_config(my_model, MQ.QuantizationConfig(**cfg))
-        q = calibrate(ref_model)
-        load_qparams(ref_model, q)
-        load_qparams(my_model, q)
-        err = compare_models(my_model, ref_model, "initialized")
-        if err is None:
-            rc, mc = R.ModelCompressor.from_pretrained_model(ref_model), M.ModelCompressor.from_pretrained_model(my_model)
-            rc.compress_model(ref_model)
-            mc.compress_model(my_model)
-            err = compare_models(my_model, ref_model, "compressed")
-        if err is None:
-            with tempfile.TemporaryDirectory() as d1, tempfile.TemporaryDirectory() as d2:
-                rc.update_config(d1)
-                mc.update_config(d2)
-                c1 = json.load(open(os.path.join(d1, "config.json")))["quantization_config"]
-                c2 = json.load(open(os.path.join(d2, "config.json")))["quantization_config"]
-                c1.pop("version", None), c2.pop("version", None)
-                if c1 != c2:
-                    err = "config.json: " + json.dumps({k: (c1.get(k), c2.get(k)) for k in set(c1) | set(c2) if c1.get(k) != c2.get(k)})[:600]
-        if err is None:
-            def back(mcomp, model):
-                try:
-                    mcomp.decompress_model(model)
-                    return None
-                except Exception as e:  # noqa: BLE001  (e.g. FP8_BLOCK with an [N, 1] scale grid: dequantize infers CHANNEL and the broadcast fails)
-                    return type(e).__name__
-
-            r_err, m_err = back(rc, ref_model), back(mc, my_model)
-            if r_err or m_err:
-                err = None if (r_err and m_err) else f"decompress_model: reference {r_err or 'ok'}, mirror {m_err or 'ok'}"
-            else:
-                err = compare_models(my_model, ref_model, "decompressed")
+        q = calibrate(my_model)
+        mine = pipeline(M, my_model, q, m_state)
+        if REF.recording:
+            rnd.setstate(st)
+            ref_model = build(rnd, seed)
+            RQ.apply_quantization_config(ref_model, RQ.QuantizationConfig(**cfg))
+            ref_stages = pipeline(R, ref_model, q, r_state)
+        err = None
+        for stage in STAGES:
+            r = REF(stage, lambda: next(ref_stages))
+            m = evaluate(lambda: next(mine))
+            if err is None and r != m:
+                err = f"{stage}: reference {r}, mirror {m}"
         checked += 1
         if err:
             bad += 1
             if bad <= 8:
                 print(f"model {case} {preset}: {err}")
     print(f"model_compressor: {checked} models checked, {bad} mismatches", flush=True)
-    sys.exit(1 if bad else 0)
+    left = REF.finish()
+    sys.exit(1 if (bad or left) else 0)
 
 
 if __name__ == "__main__":

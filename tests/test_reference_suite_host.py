@@ -1,97 +1,28 @@
 """
-The reference's OWN hot-path test files, run unmodified against this package's host mirror through the drop-in alias
-(`compat/compressed_tensors`) with the tensor-level ops backed by the CPU oracle (tests/reference_compat/oracle_patch.py).
-Only possible where the reference checkout is mounted (the build container); skipped elsewhere.  The CUDA kernels are covered by
-the `-m gpu` tests, which re-express the same files (tests/test_gpu_reference_suite.py, test_gpu_fp4.py, test_gpu_convert.py).
+The host mirror, the CPU oracle and the compressor / ModelCompressor layers against the reference, on the seeded cases of the
+differential fuzz scripts under tests/reference_compat/, compared with the reference's outcomes recorded in
+tests/golden/reference_fuzz/ (tests/reference_compat/recorded.py).  The tensor-level ops are backed by the CPU oracle
+(tests/reference_compat/oracle_patch.py); the CUDA kernels are covered by the `-m gpu` tests, which re-express the reference's own
+hot-path test files (tests/test_gpu_reference_suite.py, test_gpu_fp4.py, test_gpu_convert.py).
 """
 import os
-import re
 import subprocess
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_TESTS = "/root/reference/tests"
-
-# file -> minimum number of tests that must pass (the rest are the reference's own GPU / Triton skips)
-FILES = {
-    "test_compressors/test_pack_quant.py": 133,
-    "test_compressors/test_int_quant.py": 6,
-    "test_compressors/test_fp8_quant.py": 11,
-    "test_compressors/test_fp4_quant.py": 3,
-    "test_compressors/test_mxfp4_quant.py": 3,
-    "test_compressors/test_mxfp8_quant.py": 4,
-    "test_compressors/test_packed_asym_decompression.py": 4,
-    "test_quantization/lifecycle/test_forward.py": 35,
-    "test_quantization/lifecycle/test_enabled.py": 1,
-    "test_quantization/test_quant_args.py": 19,
-    "test_quantization/test_quant_scheme.py": 7,
-    "test_quantization/test_utils/test_helpers.py": 16,
-    "test_quantization/test_utils/test_mxfp4_utils.py": 6,
-    "test_quantization/test_utils/test_mxfp8_utils.py": 8,
-    "test_configs/test_base.py": 4,
-    "test_configs/test_infer_quant.py": 4,
-    "test_entrypoints/convert/converters/test_build_inverse_weight_maps.py": 1,
-    "test_entrypoints/convert/converters/test_modelopt_nvfp4.py": 3,
-    "test_entrypoints/convert/converters/test_autoawq.py": 7,
-    "test_entrypoints/convert/converters/test_ct_dequantizer.py": 7,
-    "test_entrypoints/convert/converters/test_fp8block_dequantizer.py": 4,
-    "test_quantization/test_quant_config.py": 12,
-    "test_compressors/model_compressors/test_model_compressor.py": 13,   # the 2 torchrun tests need 2 GPUs
-    "test_compressors/test_fp4_optimizations.py": 4,
-    "test_quantization/lifecycle/test_static_lifecycle.py": 9,
-    "test_quantization/lifecycle/test_lifecycle.py": 1,
-    "test_quantization/test_configs/test_bit_depths.py": 18,
-    "test_quantization/test_configs/test_compression_format.py": 13,
-    "test_quantization/test_configs/test_strategies.py": 18,
-    "test_quantization/test_quant_metadata.py": 1,
-    "test_transform/test_transform_args.py": 3,
-    "test_transform/test_transform_config.py": 4,
-    "test_transform/test_transform_scheme.py": 3,
-    "test_utils/test_type.py": 5,
-    "test_utils/test_helpers.py": 7,
-    "test_utils/test_safetensors_load.py": 3,
-    "test_utils/test_match.py": 60,
-}
-# deselected everywhere: tests that need the Hugging Face Hub (no network in the build container) or the reference's offload subsystem
-# (out of scope; the shim refuses loudly)
-DESELECT = "not map_to_checkpoint_names and not llama_stories and not (test_clear and True)"
-
-# one pytest process per directory of the reference's test tree (its conftest.py files are per directory); ~10 s each
-GROUPS: dict = {}
-for _path, _n in FILES.items():
-    GROUPS.setdefault(os.path.dirname(_path), []).append(_path)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="the reference checkout is only mounted in the build container")
-@pytest.mark.parametrize("group", sorted(GROUPS))
-def test_reference_files_pass_on_the_host_mirror(group):
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "tests", "reference_compat"), os.path.join(ROOT, "compat"), ROOT]))
-    paths = [os.path.join(REF_TESTS, p) for p in GROUPS[group]]
-    r = subprocess.run([sys.executable, "-m", "pytest", "-p", "oracle_patch", *paths, "-q", "-rp", "-p", "no:cacheprovider", "-k", DESELECT],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=900)
-    lines = r.stdout.strip().splitlines()
-    tail = lines[-1] if lines else r.stderr[-500:]
-    assert r.returncode == 0 and "failed" not in tail and "error" not in tail, r.stdout[-3000:]
-    for p in GROUPS[group]:
-        passed = sum(1 for line in lines if line.startswith("PASSED") and f"/{p}::" in line)
-        assert passed >= FILES[p], f"{p}: {passed} passed, expected at least {FILES[p]}\n{tail}"
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="the reference checkout is only mounted in the build container")
 def test_host_mirror_matches_the_reference_under_fuzz():
     """random QuantizationArgs / QuantizationScheme constructions and qparam computations give the same values -- or the same
-    exception type -- in the reference and in the mirror (tests/reference_compat/fuzz_host_mirror.py, ~2500 comparisons)"""
+    exception type -- in the mirror as in the reference (tests/reference_compat/fuzz_host_mirror.py, ~2500 comparisons)"""
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "reference_compat", "fuzz_host_mirror.py"), "300"],
                        capture_output=True, text=True, cwd="/tmp", timeout=600)
     lines = [line for line in r.stdout.splitlines() if "checked" in line]
     assert r.returncode == 0 and len(lines) == 3 and all(line.endswith(" 0 mismatches") for line in lines), r.stdout[-2000:] + r.stderr[-1000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="the reference checkout is only mounted in the build container")
 def test_oracle_matches_the_reference_under_fuzz():
-    """fresh random cases, beyond the committed goldens: the CPU oracle against the reference's own quantize / dequantize / fake_quantize
+    """seeded random cases, beyond the committed goldens: the CPU oracle against the reference's own quantize / dequantize / fake_quantize
     (every strategy, int 2..8 / fp8 / fp4, three dtypes) and pack / unpack functions (tests/reference_compat/fuzz_oracle.py)"""
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "reference_compat", "fuzz_oracle.py"), "200"],
                        capture_output=True, text=True, cwd="/tmp", timeout=600)
@@ -99,7 +30,6 @@ def test_oracle_matches_the_reference_under_fuzz():
     assert r.returncode == 0 and len(lines) == 2 and all(line.endswith(" 0 mismatches") for line in lines), r.stdout[-2000:] + r.stderr[-1000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="the reference checkout is only mounted in the build container")
 def test_compressor_plugins_match_the_reference_under_fuzz():
     """compress() / decompress() of every registered quantization format on random weights, schemes and strategies: same keys, dtypes,
     shapes and bits as the reference's classes (tests/reference_compat/fuzz_compressors.py; oracle-backed ops, CPU)"""
@@ -109,7 +39,6 @@ def test_compressor_plugins_match_the_reference_under_fuzz():
     assert r.returncode == 0 and len(lines) == 2 and all(" 0 mismatches" in line for line in lines), r.stdout[-2000:] + r.stderr[-1000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="the reference checkout is only mounted in the build container")
 def test_model_compressor_matches_the_reference_under_fuzz():
     """ModelCompressor end to end on random small models and presets, next to the reference's: module state dicts after
     apply_quantization_config, after compress_model and after decompress_model, and the quantization_config written to config.json
